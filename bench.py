@@ -2,7 +2,7 @@
 """Headline benchmark: VNet3d(1,2) 96^3, batch 2 per GPU, bf16 storage, forward + loss + backward
 (+ gradient all-reduce for N > 1) in voxels/second (BASELINE.json `metric`, config[1] / config[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-graph]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-graph] [--dump-outputs DIR]
 
 N > 1 is launched by the driver as ``python -m torch.distributed.run --nproc-per-node N bench.py --gpus N``
 (one rank per GPU, NCCL).  Rank 0 prints ONE JSON line.  A "step" = one pass of the hot path
@@ -297,6 +297,29 @@ def make_batch(rank: int, world: int):
     return x[sl].contiguous(), y[sl].contiguous()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(loss, dice, model):
+    """What a caller of the timed step receives: the loss, the per-step Dice and the gradient of every parameter,
+    copied to the host as float32 arrays {name: array}."""
+    import numpy as np
+    out = {"loss": loss, "dice": dice}
+    out.update({"grad." + n: p.grad for n, p in model.named_parameters()})
+    return {k: np.array(v.detach().float().cpu().numpy()) for k, v in out.items()}
+
+
+def write_outputs(directory, outputs):
+    """DIR/<name>.npy for every array; refuses more than DUMP_LIMIT_BYTES in all."""
+    import numpy as np
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"[bench] --dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_reference(args):
     """The reference's own CPU path for this metric: the oracle restatement (kind 'port') on all host cores."""
     import oracle
@@ -393,7 +416,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-variants", action="store_true", help="skip the fwd-only / optimizer / fp32 variants (N=1)")
     ap.add_argument("--workload", default="vnet3d96", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, Dice, every parameter gradient) as "
+                         "DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _capture_stdout()
     select_workload(args.workload)
     args.warmup = max(3, args.warmup)
@@ -512,11 +540,13 @@ def main():
         torch.cuda.synchronize()
         return [a.elapsed_time(b) for a, b in evs]
 
+    last_loss = [None]
+
     def resident_step():
         if use_graph:
-            graphed()                      # replays on the static (HBM-resident) input buffers
+            last_loss[0] = graphed()       # replays on the static (HBM-resident) input buffers
         else:
-            eager_step(x, y)
+            last_loss[0] = eager_step(x, y)
 
     host_losses = [torch.empty((), dtype=torch.float32).pin_memory() for _ in range(2)]
     loss_values = []
@@ -562,6 +592,11 @@ def main():
     clocks = sampler.stop()
     if sum(ms) * 1e-3 > wall * 1.02 + 1e-3:
         raise SystemExit(f"[bench] rank {rank}: inconsistent timing: event sum {sum(ms):.2f} ms > wall {wall * 1e3:.2f} ms")
+    # the e2e loop below reuses the step's static buffers: copy the last timed step's outputs first
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        dice = graphed.dice if use_graph else lossfn.last_dice()
+        outputs = step_outputs(last_loss[0], dice, model)
     e2e_loop(2)
     barrier()
     ms_e2e = e2e_loop(args.steps)
@@ -699,6 +734,8 @@ def main():
         }
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_sample()
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         _emit(line)
     if world > 1:
         del graphed                    # graphs first, then the communicator

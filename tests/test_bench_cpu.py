@@ -57,6 +57,25 @@ def test_workload_selection_and_batches():
         bench.select_workload("vnet3d96")
 
 
+def test_dump_outputs_writes_loss_dice_and_every_gradient(tmp_path):
+    import numpy as np
+    m = torch.nn.Sequential(torch.nn.Conv3d(1, 2, 3), torch.nn.GroupNorm(1, 2))
+    m(torch.randn(1, 1, 4, 4, 4)).sum().backward()
+    out = bench.step_outputs(torch.tensor(0.5), torch.tensor(0.25, dtype=torch.float64), m)
+    bench.write_outputs(str(tmp_path / "d"), out)
+    names = {"loss", "dice"} | {"grad." + n for n, _ in m.named_parameters()}
+    assert {p.name for p in (tmp_path / "d").iterdir()} == {n + ".npy" for n in names}
+    for n, p in m.named_parameters():
+        a = np.load(tmp_path / "d" / f"grad.{n}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, p.grad.numpy())
+    dice = np.load(tmp_path / "d" / "dice.npy")
+    assert dice.shape == () and dice.dtype == np.float32 and float(dice) == 0.25
+    big = {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, np.float32)}
+    with pytest.raises(SystemExit):
+        bench.write_outputs(str(tmp_path / "e"), big)
+    assert not (tmp_path / "e").exists()
+
+
 def test_b200_arm_refuses_to_run_without_a_gpu():
     """no CPU fallback: the product arm exits with an error when there is no CUDA device (SURVEY 8c, tier rule 3)"""
     if torch.cuda.is_available():

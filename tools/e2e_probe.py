@@ -1,6 +1,7 @@
 import os, sys, time, torch
-sys.path.insert(0, "/root/repo")
-os.chdir("/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+os.chdir(ROOT)
 import pytorchdeeplearing_b200 as b200
 from pytorchdeeplearing_b200.graphed import GraphedStep
 import oracle
